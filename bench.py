@@ -311,6 +311,54 @@ def cpu_baseline_quick():
 
 
 # --------------------------------------------------------------------------- CUDA arm
+PARAM_SAMPLE = 1 << 20   # fp32 master weights written by --dump-outputs (4 MB + 8 MB of float64 indices)
+DUMP_BUDGET = 64 << 20   # bytes --dump-outputs writes at most
+
+
+def dump_outputs(out_dir, eng, last):
+    """--dump-outputs: what the last timed step computed, as float32 / float64 .npy files (~28 MB at the default
+    batch, never more than DUMP_BUDGET), so two builds can be compared output for output.  The inputs are seeded, so the same arguments give the
+    same inputs on every run.  Written: the features and their lengths, the batch-mean loss and the input frame count
+    (what Speech2Text.train_step returns), the per-utterance CTC loss and the logits of that step's forward pass, and
+    a fixed, seeded sample of the parameters after its optimizer update (with the flat indices of the sample).
+    Features and logits are written for the first U utterances of the batch, U as large as the budget allows (all
+    32 at the default batch).  That step starts from the seeded initial training state (see run_own), so the features repeat bit for bit and
+    the rest differs between runs only by that one step's float-atomic reductions, amplified through the 53 bf16
+    layers (two runs of --steps 10 on a B200 at 1000 W: loss 5e-5 apart relative, sampled parameters 8e-4 absolute,
+    logits 1.6 % in relative L2 norm)."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    ws = eng._last_ws
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(0).choice(eng.master.numel(), min(PARAM_SAMPLE, eng.master.numel()),
+                                                  replace=False))
+    arrays = {
+        "feature_lengths": last["feature_lengths"].double(),
+        "loss": last["loss"].float().reshape(1),
+        "frames": last["frames"].double().reshape(1),
+        "loss_per_utterance": ws.loss.float(),
+        "params_sample": eng.master[torch.from_numpy(idx).to(eng.master.device)].float(),
+        "params_sample_index": torch.from_numpy(idx.astype(np.float64)),
+    }
+    feats, logits = last["features"], ws.logits
+    per_utt = 4 * (feats[0].numel() + logits[0].numel())
+    fixed = sum(t.numel() * t.element_size() for t in arrays.values())
+    n_utt = min(feats.shape[0], (DUMP_BUDGET - fixed - 4096) // per_utt)   # (4 KB for the .npy headers)
+    arrays.update(features=feats[:n_utt].float(), logits=logits[:n_utt].float())
+    assert sum(t.numel() * t.element_size() for t in arrays.values()) <= DUMP_BUDGET
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
+
+
+def training_state(eng):
+    """Every device buffer a training step reads and then updates: fp32 masters, gradients and optimizer slots, the
+    16-bit weight copies, the merged residual kernels, BN moving statistics, the loss-scaler / step / dropout counters."""
+    ts = [eng.master, eng.grad, eng.mom, eng.wb, eng.fstate, eng.istate] + list(eng.wcat) + list(eng.dwcat)
+    ts += list(eng.moving.values()) + [eng._opt[k] for k in ("ema", "norms", "nonfinite", "coef")]
+    return ts + [t for t in (eng.mom2, eng.grad_acc) if t is not None]
+
+
 def run_own(args):
     import numpy as np
     import torch
@@ -344,16 +392,23 @@ def run_own(args):
     model.compile()
     eng = model.engine
     dl = model.get_data_layer()
+    # the seeded initial training state; the last timed step starts from it again (see below).  One device copy made
+    # before any step, on every run so that the timed path is the same with and without --dump-outputs: ~4.7 GB of
+    # HBM per rank for Jasper 10x5 (fp32 masters, gradients and momenta, 3 x 1.33 GB, + the 0.67 GB 16-bit weights)
+    initial_state = [(t, t.clone()) for t in training_state(eng)]
 
     # the synthetic utterances come from the data layer's own in-memory generator ("synthetic:<n>:<seconds>" in
     # configs/jasper10x5_dr.py: int16 Gaussian-noise waveforms + random transcripts, SURVEY.md section 8d)
     res_targets = None
     loss_host = torch.zeros(1, dtype=torch.float32).pin_memory()
 
+    last = {}
+
     def step_resident():
         # waveforms already in HBM (dl keeps a device staging buffer): featurizer + train step
         feats, flens = dl.featurize_resident(seed=eng.step_count)
-        model.train_step({"source_tensors": [feats, flens], "target_tensors": res_targets})
+        loss, frames = model.train_step({"source_tensors": [feats, flens], "target_tensors": res_targets})
+        last.update(features=feats, feature_lengths=flens, loss=loss, frames=frames)
 
     # end to end = the call sequence a user of the plugin API makes (utils/funcs.py train loop): next(iterator) --
     # the data layer's producer thread stages the batch's HOST waveforms in pinned memory, copies them to the
@@ -409,9 +464,23 @@ def run_own(args):
         step_resident()
     barrier()
     nv0 = nvlink_counters(local) if (world > 1 and rank == 0) else None
-    ms = timed(step_resident, args.steps)
+    # The reductions of a step sum with float atomics, so two runs' training states drift apart step by step.  The
+    # last of the K timed steps therefore starts from the seeded initial state, restored between two timed windows:
+    # what it computes (--dump-outputs) depends only on the arguments, up to that one step's rounding.  That step
+    # runs at the initial weights, loss scale, scaler iteration and global step (the learning rate of step 0).  The
+    # running count of skipped (non-finite) steps, istate[4], is not part of that state: it carries over, so
+    # `skipped_steps` counts every step of the run.
+    ms = timed(step_resident, args.steps - 1) if args.steps > 1 else 0.0
+    if args.steps > 0:
+        skipped_so_far = int(eng.istate[4])
+        for t, t0 in initial_state:
+            t.copy_(t0)
+        eng.istate[4] = skipped_so_far
+        ms += timed(step_resident, 1)
     nv1 = nvlink_counters(local) if nv0 is not None else None
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, last)
 
     # roofline of the dominant kernel family (tcgen05 implicit-GEMM conv): per-launch CUDA-event
     # timing of every conv launch of instrumented steps run right after the timed region
@@ -497,6 +566,8 @@ def main():
     ap.add_argument("--no_cpu_baseline", action="store_true")
     ap.add_argument("--no_augmentation", action="store_true",
                     help="A/B measurement without the recipe's speed perturbation (fixed 15 s utterances)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

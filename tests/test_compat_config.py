@@ -14,8 +14,8 @@ compat.install()
 
 from open_seq2seq.utils.utils import (check_params, flatten_dict, get_base_config, nest_dict,  # noqa: E402
                                       nested_update)
+from tests.refpins import example_config  # noqa: E402
 
-REF_CFG = "/root/reference/example_configs/speech2text/jasper10x5_LibriSpeech_nvgrad.py"
 OWN_CFG = os.path.join(ROOT, "configs", "jasper10x5_dr.py")
 
 
@@ -31,14 +31,9 @@ def test_own_jasper_config_loads_with_cli_overrides():
     assert args.mode == "train"
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CFG), reason="reference checkout not present (GPU box)")
-def test_reference_jasper_config_loads_unchanged_and_matches_own_config():
-    cwd = os.getcwd()
-    os.chdir("/root/reference")  # the reference config uses a path relative to its repo root
-    try:
-        _, ref, ref_model, ref_mod = get_base_config(["--config_file=" + REF_CFG, "--mode=train"])
-    finally:
-        os.chdir(cwd)
+def test_reference_jasper_config_loads_unchanged_and_matches_own_config(tmp_path):
+    ref_cfg = example_config("jasper10x5_LibriSpeech_nvgrad.py", tmp_path)
+    _, ref, ref_model, ref_mod = get_base_config(["--config_file=" + ref_cfg, "--mode=train"])
     _, own, own_model, own_mod = get_base_config(["--config_file=" + OWN_CFG, "--mode=train"])
     assert ref_model.__name__ == own_model.__name__ == "Speech2Text"
     assert ref["encoder_params"]["convnet_layers"] == own["encoder_params"]["convnet_layers"]
@@ -55,15 +50,17 @@ def test_reference_jasper_config_loads_unchanged_and_matches_own_config():
     assert ref_mod["train_params"]["data_layer_params"]["max_duration"] == 16.7
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CFG), reason="reference checkout not present (GPU box)")
 @pytest.mark.parametrize("name", ["jasper10x5_LibriSpeech_nvgrad.py", "jasper10x5_LibriSpeech_nvgrad_masks.py",
                                   "w2lplus_large_8gpus_mp.py", "jasper-Mini-for-Jetson.py"])
-def test_other_reference_speech_configs_import_through_the_shim(name):
-    path = os.path.join("/root/reference/example_configs/speech2text", name)
-    if not os.path.exists(path):
-        pytest.skip("config not in this checkout")
-    _, cfg, model, _ = get_base_config(["--config_file=" + path, "--mode=train"])
+def test_other_reference_speech_configs_import_through_the_shim(name, tmp_path):
+    from tests.refpins import config_imports, import_names
+    imports = config_imports(name)
+    bound = import_names(imports)          # every name the config imports resolves through the drop-in packages
+    assert "Speech2Text" in bound and len(bound) == len(imports)
+    path = example_config(name, tmp_path)
+    _, cfg, model, mod = get_base_config(["--config_file=" + path, "--mode=train"])
     assert model.__name__ == "Speech2Text" and "convnet_layers" in cfg["encoder_params"]
+    assert all(mod[k] is v for k, v in bound.items())
 
 
 def test_check_params_rules_and_errors():
@@ -130,12 +127,11 @@ def test_optimizer_kwargs_from_jasper_params():
     assert kw["loss_scaling"] is True
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CFG), reason="reference checkout not present (GPU box)")
-def test_optimizer_and_data_layer_kwargs_from_reference_w2lplus_config():
+def test_optimizer_and_data_layer_kwargs_from_reference_w2lplus_config(tmp_path):
     """example_configs/speech2text/w2lplus_large_8gpus_mp.py unchanged: Momentum + poly_decay + LARC + an L2
     regulariser + the default (python_speech_features) feature backend all map onto built pieces."""
     from open_seq2seq.optimizers.optimizers import optimizer_engine_kwargs
-    path = "/root/reference/example_configs/speech2text/w2lplus_large_8gpus_mp.py"
+    path = example_config("w2lplus_large_8gpus_mp.py", tmp_path)
     _, cfg, _, mod = get_base_config(["--config_file=" + path, "--mode=train"])
     kw = optimizer_engine_kwargs(cfg, last_step=2000)
     assert kw["algo"] == "momentum" and kw["momentum"] == 0.9
@@ -173,7 +169,7 @@ def test_benchmark_flag_rewrites_the_train_config_like_the_reference():
     check_params(train_cfg, Speech2Text.get_required_params(), Speech2Text.get_optional_params())
 
 
-def test_nothing_in_the_headline_config_is_silently_ignored():
+def test_nothing_in_the_headline_config_is_silently_ignored(tmp_path):
     """The reference's jasper10x5_LibriSpeech_nvgrad.py trains with speed perturbation (train_params
     augmentation :199-201); accepted-but-unimplemented options must raise, implemented ones must reach the
     engine / data layer."""
@@ -185,9 +181,8 @@ def test_nothing_in_the_headline_config_is_silently_ignored():
     _, cfg, _, mod = get_base_config(["--config_file=" + OWN_CFG])
     aug = mod["train_params"]["data_layer_params"]["augmentation"]
     assert aug == {"speed_perturbation_ratio": [0.9, 1.0, 1.1]}
-    if os.path.exists(REF_CFG):
-        _, _, _, ref_mod = get_base_config(["--config_file=" + REF_CFG])
-        assert ref_mod["train_params"]["data_layer_params"]["augmentation"] == aug
+    _, _, _, ref_mod = get_base_config(["--config_file=" + example_config("jasper10x5_LibriSpeech_nvgrad.py", tmp_path)])
+    assert ref_mod["train_params"]["data_layer_params"]["augmentation"] == aug
     base = dict(cfg["data_layer_params"], mode="train", batch_size=2, dataset_files=["synthetic:4:1.0"])
     dl = Speech2TextDataLayer(dict(base, augmentation=dict(aug, noise_level_min=-90, noise_level_max=-46)), None, 1, 0)
     rs = np.random.RandomState(0)
@@ -236,11 +231,10 @@ def test_nothing_in_the_headline_config_is_silently_ignored():
         resolve_initializer({"initializer": lambda **kw: None}, {}, "x")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CFG), reason="reference checkout not present (GPU box)")
-def test_quartznet_config_matches_the_reference_and_sep_conv_topology_builds_on_paper():
+def test_quartznet_config_matches_the_reference_and_sep_conv_topology_builds_on_paper(tmp_path):
     """configs/quartznet15x5.py == example_configs/speech2text/quartznet15x5_LibriSpeech.py (layers, optimizer,
     lr policy, spec-augment); sep_conv1d layers map to variables with tf.layers.separable_conv1d's names."""
-    ref_path = "/root/reference/example_configs/speech2text/quartznet15x5_LibriSpeech.py"
+    ref_path = example_config("quartznet15x5_LibriSpeech.py", tmp_path)
     _, ref, _, rmod = get_base_config(["--config_file=" + ref_path, "--mode=train"])
     _, own, _, omod = get_base_config(["--config_file=" + os.path.join(ROOT, "configs", "quartznet15x5.py"), "--mode=train"])
     assert ref["encoder_params"]["convnet_layers"] == own["encoder_params"]["convnet_layers"]
@@ -256,7 +250,6 @@ def test_quartznet_config_matches_the_reference_and_sep_conv_topology_builds_on_
     assert "conv25/res_bn/gamma" in p and "conv21/kernel" not in p
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CFG), reason="reference checkout not present (GPU box)")
 @pytest.mark.parametrize("name,optimizer,policy,larc,aug", [
     ("jasper10x5_LibriSpeech_nvgrad_masks.py", "NovoGrad", "poly_decay", True, True),
     ("jasper-Mini-for-Jetson.py", "NovoGrad", "poly_decay", True, True),
@@ -282,7 +275,7 @@ def test_create_model_dry_run_of_every_tdnn_example_config(monkeypatch, golden_d
         return orig(self, *a, **kw)
     monkeypatch.setattr(E.JasperEngine, "__init__", on_cpu)
     toy = os.path.join(golden_dir, "toy_speech_data")
-    path = os.path.join("/root/reference/example_configs/speech2text", name)
+    path = example_config(name, tmp_path)
     args, cfg, model, module = get_base_config(["--config_file=" + path, "--mode=train_eval"])
     module = dict(module)
     for k in ("train_params", "eval_params"):

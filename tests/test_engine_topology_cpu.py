@@ -116,10 +116,6 @@ def test_gradient_buckets_tile_the_flat_buffer_and_split_into_aligned_rank_slice
                     assert lo == sl[r - 1][1]
 
 
-REF_SPEECH_CONFIGS = "/root/reference/example_configs/speech2text"
-
-
-@pytest.mark.skipif(not __import__("os").path.isdir(REF_SPEECH_CONFIGS), reason="reference checkout not present")
 @pytest.mark.parametrize("name,layers,params,sep", [
     ("jasper10x5_LibriSpeech_nvgrad_masks.py", 53, 332632349, False),   # (same encoder as ..._nvgrad.py)
     ("jasper-Mini-for-Jetson.py", 33, 8192733, True),
@@ -129,14 +125,14 @@ REF_SPEECH_CONFIGS = "/root/reference/example_configs/speech2text"
     ("w2lplus_large_8gpus.py", 18, 106496285, False),
     ("w2lplus_large_8gpus_mp.py", 18, 106496285, False),
 ])
-def test_every_tdnn_example_config_of_the_reference_builds_an_engine(cpu_engine, name, layers, params, sep):
+def test_every_tdnn_example_config_of_the_reference_builds_an_engine(cpu_engine, name, layers, params, sep, tmp_path):
     """All TDNNEncoder configs under example_configs/speech2text load unchanged through the compat package and
     their encoder params (activation, normalisation, initializer, conv / sep_conv layers, residual topologies,
     channel widths) map onto a JasperEngine: number of trainable variables as a regression value."""
-    import os
     from open_seq2seq.encoders import TDNNEncoder
     from open_seq2seq.utils.utils import get_base_config
-    _, cfg, model, _ = get_base_config(["--config_file=" + os.path.join(REF_SPEECH_CONFIGS, name), "--mode=train"])
+    from tests.refpins import example_config
+    _, cfg, model, _ = get_base_config(["--config_file=" + example_config(name, tmp_path), "--mode=train"])
     assert model.__name__ == "Speech2Text" and cfg["encoder"] is TDNNEncoder
     kw = TDNNEncoder(dict(cfg["encoder_params"]), None, mode="train").engine_kwargs()
     nf = cfg.get("data_layer_params", {}).get("num_audio_features", 64)

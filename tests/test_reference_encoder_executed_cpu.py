@@ -1,4 +1,4 @@
-"""The reference's OWN encoder code executed here (CPU, build container only) against the oracle.
+"""The reference's OWN encoder code, executed and stored, against the oracle (CPU tests).
 
 `TDNNEncoder._encode` (encoders/tdnn_encoder.py:87-265) and `conv_bn_actv / conv_bn_res_bn_actv`
 (parts/cnns/conv_blocks.py:61-232) are graph BUILDERS: every number they produce comes from a handful of TensorFlow
@@ -8,11 +8,13 @@ transpose / reduce_max / mod / constant`, `tf.nn.dropout`) written from TensorFl
 (SAME padding `out = ceil(T / s)`, `pad = max((out - 1) s + (K - 1) d + 1 - T, 0)`, the smaller half on the left;
 training-mode batch normalisation over every axis but the channel axis, biased variance; depth multiplier 1), with
 the variables looked up BY THE NAME TensorFlow would give them.  The reference's own source, loaded by path / compiled
-from `/root/reference` (never copied), then builds the encoder: which layer is called with which input, in which
+from a checkout of it (never copied), then builds the encoder: which layer is called with which input, in which
 order, where the masks are applied and refreshed, how the lengths shrink, which residual sources feed which block
 through which 1x1 convolution and batch norm, under which variable names.  The oracle (`oracle/torch_twin.py`
 tdnn_encode -- what every GPU parity test compares with, and whose variable set the engine reproduces) must give the
-same output, the same lengths, and use exactly the same variables.  Skipped on the GPU box.
+same output, the same lengths, and use exactly the same variables.  The reference's outputs are stored under
+tests/golden/reference/reference_encoder.json (tests/refpins.py; OS2S_REFERENCE_ROOT re-runs the reference and
+rewrites them).
 """
 import ast
 import importlib.util
@@ -26,10 +28,10 @@ import torch
 import torch.nn.functional as F
 
 from oracle import torch_twin as TT
+from tests import refpins as RP
 from tests.common_cfg import MINI_JASPER, MINI_QUARTZ
 
-REF_ROOT = "/root/reference/open_seq2seq"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_ROOT), reason="reference checkout not present (GPU box)")
+PINS = RP.Pins("reference_encoder")
 
 
 class EagerTF(object):
@@ -111,7 +113,7 @@ class EagerTF(object):
     constant = staticmethod(lambda v: v)
 
 
-def _reference_encoder(tf):
+def _reference_encoder(root, tf):
     """conv_blocks.py loaded by path with `tensorflow` = the eager stand-in, then TDNNEncoder._encode compiled from
     its source into a namespace that holds those block functions."""
     pk = {n: types.ModuleType(n) for n in ("_refpkg", "_refpkg.parts", "_refpkg.parts.cnns", "_refpkg.parts.cnns.tcn")}
@@ -125,7 +127,7 @@ def _reference_encoder(tf):
     sys.modules.update(stand)
     try:
         spec = importlib.util.spec_from_file_location("_refpkg.parts.cnns.conv_blocks",
-                                                      os.path.join(REF_ROOT, "parts/cnns/conv_blocks.py"))
+                                                      os.path.join(root, "open_seq2seq/parts/cnns/conv_blocks.py"))
         blocks = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(blocks)
     finally:
@@ -139,7 +141,7 @@ def _reference_encoder(tf):
     class Speech2TextDataLayer(object):
         def __init__(self, params):
             self.params = params
-    path = os.path.join(REF_ROOT, "encoders/tdnn_encoder.py")
+    path = os.path.join(root, "open_seq2seq/encoders/tdnn_encoder.py")
     cls = next(n for n in ast.parse(open(path).read()).body if isinstance(n, ast.ClassDef) and n.name == "TDNNEncoder")
     fn = next(n for n in cls.body if isinstance(n, ast.FunctionDef) and n.name == "_encode")
     ns = {"tf": tf, "Speech2TextDataLayer": Speech2TextDataLayer}
@@ -180,24 +182,28 @@ def test_oracle_encoder_equals_the_executed_reference_encoder(name, layers, use_
         T = -(-max(lens) // 16) * 16
         x = torch.randn(len(lens), T, F_in, dtype=torch.float64)
         x = x * TT.sequence_mask(lens_t, T, x.dtype)         # the data layer pads with zeros
-        tf = EagerTF(params)
-        encode, DataLayer = _reference_encoder(tf)
-        me = types.SimpleNamespace(
-            params={"convnet_layers": layers, "dropout_keep_prob": 1.0, "activation_fn": torch.relu,
-                    "use_conv_mask": use_conv_mask, "data_format": "channels_last", "normalization": "batch_norm",
-                    "bn_momentum": 0.9, "bn_epsilon": 1e-3},
-            _mode="train",
-            _model=types.SimpleNamespace(get_data_layer=lambda: DataLayer({"backend": "librosa", "pad_to": 16})))
-        want = encode(me, {"source_tensors": [x, lens_t.clone()]})
+
+        def reference(root):
+            tf = EagerTF(params)
+            encode, DataLayer = _reference_encoder(root, tf)
+            me = types.SimpleNamespace(
+                params={"convnet_layers": layers, "dropout_keep_prob": 1.0, "activation_fn": torch.relu,
+                        "use_conv_mask": use_conv_mask, "data_format": "channels_last", "normalization": "batch_norm",
+                        "bn_momentum": 0.9, "bn_epsilon": 1e-3},
+                _mode="train",
+                _model=types.SimpleNamespace(get_data_layer=lambda: DataLayer({"backend": "librosa", "pad_to": 16})))
+            want = encode(me, {"source_tensors": [x, lens_t.clone()]})
+            return {"src_length": want["src_length"], "outputs": want["outputs"], "used": sorted(tf.used)}
+        want = PINS("encoder/%s/mask=%s/%s" % (name, use_conv_mask, lens), reference)
         got, got_len = TT.tdnn_encode(x, lens_t, layers, params, training=True, bn_eps=1e-3,
                                       use_conv_mask=use_conv_mask)
-        assert torch.equal(want["src_length"], got_len), name
-        assert want["outputs"].shape == got.shape
-        err = float((want["outputs"] - got).abs().max() / want["outputs"].abs().max())
+        assert RP.equal(got_len, want["src_length"]), name
+        assert want["outputs"].shape == tuple(got.shape)
+        err = RP.max_dev(got, want["outputs"]) / want["outputs"].absmax
         assert err < 1e-10, (name, lens, err)
         # exactly the encoder's variables were read, each once, under TensorFlow's names
         enc_vars = sorted(k for k in params if not k.startswith("fc/"))
-        assert sorted(tf.used) == enc_vars, (set(enc_vars) ^ set(tf.used))
+        assert want["used"] == enc_vars, (set(enc_vars) ^ set(want["used"]))
 
 
 def _compile_from(path, cls_name, fn_name, ns):
@@ -270,28 +276,33 @@ def test_oracle_forward_loss_equals_the_executed_reference_encoder_decoder_and_l
     y = torch.zeros(4, 11, dtype=torch.int64)
     for b in range(4):
         y[b, :y_len[b]] = torch.randint(0, V - 1, (int(y_len[b]),))
-    tf = EagerTFHead(params, {"fully_connected": "fc"})
-    encode, DataLayer = _reference_encoder(tf)
-    monkeypatch.setattr(torch.Tensor, "get_shape", lambda t: types.SimpleNamespace(as_list=lambda: list(t.shape)),
-                        raising=False)
-    me = types.SimpleNamespace(
-        params={"convnet_layers": layers, "dropout_keep_prob": 1.0, "activation_fn": torch.relu, "use_conv_mask": True,
-                "data_format": "channels_last", "normalization": "batch_norm", "bn_momentum": 0.9, "bn_epsilon": 1e-3,
-                "tgt_vocab_size": V},
-        _mode="train", _mask_nan=True,
-        _model=types.SimpleNamespace(get_data_layer=lambda: DataLayer({"backend": "librosa", "pad_to": 16})))
-    enc = encode(me, {"source_tensors": [x, lens_t.clone()]})
-    decode = _compile_from(os.path.join(REF_ROOT, "decoders/fc_decoders.py"), "FullyConnectedTimeDecoder", "_decode",
-                           {"tf": tf})
-    dec = decode(me, {"encoder_output": enc})
-    ns = {"tf": tf}
-    _compile_from(os.path.join(REF_ROOT, "utils/utils.py"), None, "mask_nans", ns)
-    _compile_from(os.path.join(REF_ROOT, "losses/ctc_loss.py"), None, "dense_to_sparse", ns)
-    compute = _compile_from(os.path.join(REF_ROOT, "losses/ctc_loss.py"), "CTCLoss", "_compute_loss", ns)
-    want = compute(me, {"decoder_output": dec, "target_tensors": [y, y_len]})
+
+    def reference(root):
+        tf = EagerTFHead(params, {"fully_connected": "fc"})
+        encode, DataLayer = _reference_encoder(root, tf)
+        monkeypatch.setattr(torch.Tensor, "get_shape", lambda t: types.SimpleNamespace(as_list=lambda: list(t.shape)),
+                            raising=False)
+        me = types.SimpleNamespace(
+            params={"convnet_layers": layers, "dropout_keep_prob": 1.0, "activation_fn": torch.relu,
+                    "use_conv_mask": True, "data_format": "channels_last", "normalization": "batch_norm",
+                    "bn_momentum": 0.9, "bn_epsilon": 1e-3, "tgt_vocab_size": V},
+            _mode="train", _mask_nan=True,
+            _model=types.SimpleNamespace(get_data_layer=lambda: DataLayer({"backend": "librosa", "pad_to": 16})))
+        enc = encode(me, {"source_tensors": [x, lens_t.clone()]})
+        src = os.path.join(root, "open_seq2seq")
+        decode = _compile_from(os.path.join(src, "decoders/fc_decoders.py"), "FullyConnectedTimeDecoder", "_decode",
+                               {"tf": tf})
+        dec = decode(me, {"encoder_output": enc})
+        ns = {"tf": tf}
+        _compile_from(os.path.join(src, "utils/utils.py"), None, "mask_nans", ns)
+        _compile_from(os.path.join(src, "losses/ctc_loss.py"), None, "dense_to_sparse", ns)
+        compute = _compile_from(os.path.join(src, "losses/ctc_loss.py"), "CTCLoss", "_compute_loss", ns)
+        loss = compute(me, {"decoder_output": dec, "target_tensors": [y, y_len]})
+        return {"src_length": dec["src_length"], "logits": dec["logits"], "loss": float(loss), "used": sorted(tf.used)}
+    want = PINS("forward_loss/%d_layers" % len(layers), reference)
     got, logits, out_len = TT.forward_loss(params, layers, x, lens_t, y, y_len, training=True)
-    assert torch.equal(dec["src_length"], out_len)
-    assert dec["logits"].shape == logits.shape                     # [T', B, V]
-    assert float((dec["logits"] - logits).abs().max() / logits.abs().max()) < 1e-10
-    assert abs(float(want) - float(got)) < 1e-4 * abs(float(want))  # (the twin evaluates the CTC lattice in fp32)
-    assert sorted(tf.used) == sorted(params)
+    assert RP.equal(out_len, want["src_length"])
+    assert want["logits"].shape == tuple(logits.shape)              # [T', B, V]
+    assert RP.max_dev(logits, want["logits"]) / want["logits"].absmax < 1e-10
+    assert abs(want["loss"] - float(got)) < 1e-4 * abs(want["loss"])  # (the twin evaluates the CTC lattice in fp32)
+    assert want["used"] == sorted(params)

@@ -1,10 +1,10 @@
 """Write tests/golden/reference_augmentation_draws.json from the reference's OWN augment_audio_signal
-(open_seq2seq/data/speech2text/speech_utils.py:225-268), executed in the build container (the GPU box has no
-/root/reference): for seeded global np.random streams, the output length and the drawn noise level of every call.
+(open_seq2seq/data/speech2text/speech_utils.py:225-268), executed from a checkout of the reference: for seeded
+global np.random streams, the output length and the drawn noise level of every call.
 The reference module is loaded by path with resampy replaced by the oracle's restatement (only the LENGTH of its
 result enters the fixture); see tests/test_reference_executed_cpu.py.
 
-    python tools/make_golden_reference_draws.py
+    python tools/make_golden_reference_draws.py <checkout of NVIDIA/OpenSeq2Seq>
 """
 import json
 import os
@@ -25,7 +25,7 @@ AUGS = [
 
 
 def main():
-    ref = load_reference_speech_utils()
+    ref = load_reference_speech_utils(sys.argv[1])
     n, sr = 23456, 16000
     cases = []
     for aug in AUGS:
@@ -47,7 +47,7 @@ def main():
                           "noise_level_db": drawn[0] if drawn else None})
     path = os.path.join(ROOT, "tests", "golden", "reference_augmentation_draws.json")
     with open(path, "w") as f:
-        json.dump({"source": "/root/reference/open_seq2seq/data/speech2text/speech_utils.py:225-268 executed by "
+        json.dump({"source": "open_seq2seq/data/speech2text/speech_utils.py:225-268 executed by "
                              "tools/make_golden_reference_draws.py", "n_samples": n, "sample_freq": sr, "cases": cases},
                   f, indent=1)
     print(path, len(cases), "cases")
